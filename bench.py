@@ -5,11 +5,11 @@ num_envs = 64 per rank, T = 128, ppo_epoch = 2, num_mini_batch = 2, synthetic ob
 
 One "step" = one learner iteration on a full rollout: RolloutStorage.compute_returns (GAE) +
 PPO.update (2 epochs x 2 minibatches of 4096 frames: forward, backward, [all-reduce], clip,
-Adam).  value = world * T * N / t_step  (the reference's perf/fps definition,
+Adam), each timed step from the same policy and optimizer state.  value = world * T * N / t_step  (the reference's perf/fps definition,
 habitat-baselines/habitat_baselines/rl/ppo/ppo_trainer.py:595-598, learner part).
 
     python bench.py --gpus 1 --steps K --warmup W           # this repo's sm_100a path
-    python bench.py --impl reference ...                     # the UNMODIFIED reference classes (baseline/_ref) on the CPU
+    python bench.py --impl reference ...                     # the UNMODIFIED reference classes (oracle/_ref) on the CPU
     python bench.py --impl torch_cuda ...                    # ... and on CUDA (TF32 cuDNN, cudnn.benchmark; DDP + NCCL at N > 1)
     torchrun --nproc-per-node N bench.py --gpus N ...        # one rank per GPU, NCCL
 
@@ -174,7 +174,7 @@ def _ref_kwargs():
 
 
 def _make_cpu_learner(T=CPU_SAMPLE["T"], N=CPU_SAMPLE["N"]):
-    """The UNMODIFIED reference (baseline/_ref or /root/reference through the import shim): RolloutStorage.compute_returns
+    """The UNMODIFIED reference (oracle/_ref through the import shim): RolloutStorage.compute_returns
     + PPO.update on device="cpu" -- the reference's own CPU PPO path."""
     from oracle.ref_learner import ReferenceLearner
 
@@ -307,6 +307,35 @@ def _config(n):
 # ---------------------------------------------------------------------------------------------
 # hb200 arm
 # ---------------------------------------------------------------------------------------------
+class LearnerState:
+    """What one learner step reads besides the rollout: the policy's parameters and buffers (RunningMeanAndVar), the
+    Adam moments and step count, and the CPU generator that data_generator's minibatch split draws from.  The timed steps
+    each start from the state captured before warm-up, so they compute from the same inputs in every run: the gradient
+    kernels accumulate with atomics, and a state carried from step to step would drift apart between runs by far more
+    than one step's rounding."""
+
+    def __init__(self, policy, optimizer):
+        self.policy, self.opt = policy, optimizer
+        flat = optimizer._bind()
+        self.params = flat["params"].clone()
+        self.buffers = [b.detach().clone() for b in policy.buffers()]
+        self.m, self.v, self.step = optimizer._m.clone(), optimizer._v.clone(), optimizer._step
+        self.rng = torch.get_rng_state()
+
+    @torch.no_grad()
+    def restore(self):
+        self.opt._bind()["params"].copy_(self.params)
+        for b, s in zip(self.policy.buffers(), self.buffers):
+            b.copy_(s)
+        self.opt._m.copy_(self.m)
+        self.opt._v.copy_(self.v)
+        self.opt._step = self.step
+        for st in self.opt.state.values():
+            st["step"].fill_(float(self.step))
+        self.policy.mark_weights_changed()
+        torch.set_rng_state(self.rng)
+
+
 def run_hb200(args):
     import habitat_lab_b200 as hb
     from habitat_lab_b200 import ops
@@ -349,29 +378,42 @@ def run_hb200(args):
             torch.distributed.barrier()
         torch.cuda.synchronize()
 
-    def timed(fn, steps):
+    def timed(fn, steps, before_each=None):
+        """device time of `steps` calls of fn; with before_each, the sum over the calls alone (what before_each
+        enqueues between them is not counted)"""
         barrier()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
+        n_ev = steps if before_each is not None else 1
+        ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(n_ev)]
         out = None
-        for _ in range(steps):
-            out = fn()
-        e1.record()
+        if before_each is None:
+            ev[0][0].record()
+            for _ in range(steps):
+                out = fn()
+            ev[0][1].record()
+        else:
+            for e0, e1 in ev:
+                before_each()
+                e0.record()
+                out = fn()
+                e1.record()
         barrier()
-        ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
+        ms = torch.tensor([sum(e0.elapsed_time(e1) for e0, e1 in ev)], device=dev)
         if world > 1:
             torch.distributed.all_reduce(ms, op=torch.distributed.ReduceOp.MAX)
         return ms.item(), out
 
+    start = LearnerState(policy, ppo.optimizer)   # every timed step starts from here
     for _ in range(max(args.warmup, 3)):
         learner_step()
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
     l0 = lib.hb200_launch_count()
-    ms, metrics = timed(learner_step, args.steps)
+    ms, metrics = timed(learner_step, args.steps, before_each=start.restore)
     launches = lib.hb200_launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:   # before the e2e leg below trains the policy further
+        dump_outputs(args.dump_outputs, metrics, st.buffers["returns"], policy)
     frames = world * T * N * args.steps
     value = frames / (ms * 1e-3)
     cross_rank = cross_rank_equality(policy, dev, world) if world > 1 else None
@@ -437,7 +479,7 @@ def run_hb200(args):
             torch_cuda = torch_cuda_measure(dev, world, st.buffers, next_value, args.steps, args.warmup, seed=100)
             torch_cuda["hb200_over_torch_cuda"] = value / torch_cuda["value"]
             torch_cuda["hb200_e2e_over_torch_cuda"] = e2e_value / torch_cuda["value"]
-        except Exception as e:   # e.g. baseline/_ref missing on this box: report, never lose the hb200 line
+        except Exception as e:   # e.g. oracle/_ref not installed: report, never lose the hb200 line
             torch_cuda = {"unavailable": repr(e)[:300]}
     line = None
     if rank == 0:
@@ -621,6 +663,30 @@ def run_sweep(args):
            "peaks": {"hbm_gbs": peaks["hbm"], "bf16_tflops_sustained": peaks["bf16_sustained"], "source": peaks["src"]},
            "rows": rows, "data": "synthetic"})
 
+
+
+DUMP_MAX_ELEMS = 12 << 20   # per array: 48 MB of float32, so that one policy state plus the small outputs stay under 64 MB
+
+
+def dump_outputs(out_dir, metrics, returns, policy):
+    """What the last timed learner step produced, for comparing two builds output for output: every learner metric
+    PPO.update returned (`metric_<key>.npy`, float64), the GAE returns left in the rollout storage (`returns.npy`) and
+    every floating-point tensor of the updated policy's state_dict, flattened and concatenated in state_dict order
+    (`policy_state.npy`, float32).  An array above DUMP_MAX_ELEMS is replaced by the elements at a fixed, seeded set of
+    positions (`<name>_sample.npy`), the same positions for the same array size.  Every timed step starts from the same
+    state (LearnerState), so two runs with the same arguments differ only by the rounding of the atomic gradient sums."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {f"metric_{k}": np.float64(v) for k, v in metrics.items()}
+    arrays["returns"] = returns.detach().float().cpu().numpy()
+    state = [t.detach().float().flatten() for t in policy.state_dict().values() if t.is_floating_point()]
+    arrays["policy_state"] = torch.cat(state).cpu().numpy()
+    for name, a in arrays.items():
+        if a.size > DUMP_MAX_ELEMS:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))
+            name, a = f"{name}_sample", a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def cross_rank_equality(policy, dev, world):
@@ -857,7 +923,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-torch-cuda", action="store_true", help="skip the reference PyTorch-CUDA competitor leg")
     ap.add_argument("--sweep", action="store_true", help="BASELINE configs[4]: minibatch-size sweep (1 GPU), one JSON line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed learner step computed as DIR/<name>.npy (hb200 arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.sweep or args.impl != "hb200"):
+        ap.error("--dump-outputs applies to the hb200 arm only")
     select_workload(args.config)
     if args.sweep:
         return run_sweep(args)

@@ -1,5 +1,5 @@
 """TEST / BASELINE INFRASTRUCTURE ONLY -- the UNMODIFIED reference learner (habitat_baselines classes imported through
-oracle/ref_shim.py from /root/reference or its verbatim copy under baseline/_ref/) wired up the way
+oracle/ref_shim.py from the install under oracle/_ref/) wired up the way
 `PPOTrainer._update_agent` drives it (habitat-baselines/habitat_baselines/rl/ppo/ppo_trainer.py:484-523):
 
     rollouts.compute_returns(next_value, use_gae, gamma, tau)   # common/rollout_storage.py:174-205

@@ -1,13 +1,13 @@
 """TEST INFRASTRUCTURE ONLY -- import shim that lets the *unmodified* reference
-hot-path modules under /root/reference load in this container.
+hot-path modules (installed under oracle/_ref by oracle/install_reference.py) load here.
 
 habitat-lab's packages cannot be imported as packages here (gym, omegaconf,
 hydra, habitat_sim ... are absent, and ``habitat_baselines/__init__.py``
 imports every trainer).  The hot-path files themselves contain no arithmetic
 outside torch/numpy, so they load verbatim once ``sys.modules`` is pre-seeded
 with arithmetic-free stubs (SURVEY.md section 8c).  Nothing in here is product code:
-only ``tests/golden/make_golden.py`` (fixture generation, run in the build
-container) and CPU tests that are skipped when /root/reference is absent use it.
+``tests/golden/make_golden.py`` (fixture generation), bench.py's reference
+arms and the reference arm's contract test use it.
 """
 from __future__ import annotations
 
@@ -22,15 +22,8 @@ _REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _pick_root() -> str:
-    """/root/reference in the build container; on the GPU box (where it does not exist) the verbatim copy that
-    baseline/install_reference.py placed under baseline/_ref/ (git-ignored, shipped with the snapshot)."""
-    env = os.environ.get("HB200_REFERENCE_ROOT")
-    if env:
-        return env
-    for cand in ("/root/reference", os.path.join(_REPO, "baseline", "_ref")):
-        if os.path.isdir(os.path.join(cand, "habitat-baselines", "habitat_baselines")):
-            return cand
-    return "/root/reference"
+    """HB200_REFERENCE_ROOT when set, else the install oracle/install_reference.py made under oracle/_ref/ (git-ignored)."""
+    return os.environ.get("HB200_REFERENCE_ROOT") or os.path.join(_REPO, "oracle", "_ref")
 
 
 REFERENCE_ROOT = _pick_root()

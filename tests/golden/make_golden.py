@@ -1,7 +1,8 @@
-"""Generates tests/golden/*.pt by running the UNMODIFIED reference classes (imported from
-/root/reference through oracle/ref_shim.py) on recipe inputs.  Run in the build container only:
+"""Generates tests/golden/*.pt by running the UNMODIFIED reference classes (installed under
+oracle/_ref by build(), imported through oracle/ref_shim.py) on recipe inputs.  Run where the
+reference is installed:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py [case ...]
 
 The fixtures hold only small outputs (losses, per-frame values, per-tensor gradient norms ...);
 inputs and weights are regenerated from seeds by tests/golden/recipe.py.
@@ -138,10 +139,52 @@ def _next_cases(R, only):
 
 
 
+def _ppo_loss_case(R):
+    """PPO._update_from_batch's loss section (rl/ppo/ppo.py:164-299) on random features through linear heads: the
+    inputs, the head weights and the metrics the reference logs, for tests/test_oracle.py."""
+    torch.manual_seed(0)
+    B, A = 64, 4
+    feats = torch.randn(B, 512)
+
+    class FakeAC(torch.nn.Module):
+        def __init__(self):
+            super().__init__()
+            self.lin = torch.nn.Linear(512, A)
+            self.val = torch.nn.Linear(512, 1)
+
+        def evaluate_actions(self, obs, h, pa, m, actions, info):
+            dist = torch.distributions.Categorical(logits=self.lin(obs))
+            return self.val(obs), dist.log_prob(actions.squeeze(-1)).unsqueeze(-1), dist.entropy().unsqueeze(-1), h, {}
+
+        def policy_parameters(self):
+            return self.parameters()
+
+        def aux_loss_parameters(self):
+            return {}
+
+    ac = FakeAC()
+    ppo = R.PPO(ac, clip_param=0.2, ppo_epoch=1, num_mini_batch=1, value_loss_coef=0.5, entropy_coef=0.01, lr=0.0,
+                eps=1e-5, max_grad_norm=0.2, use_clipped_value_loss=True, use_normalized_advantage=False)
+    batch = dict(observations=feats, recurrent_hidden_states=None, prev_actions=None, masks=None,
+                 actions=torch.randint(0, A, (B, 1)), action_log_probs=torch.randn(B, 1) * 0.3 - 1.4,
+                 advantages=torch.randn(B, 1), value_preds=torch.randn(B, 1) * 0.3, returns=torch.randn(B, 1))
+    heads = {k: v.detach().clone() for k, v in ac.state_dict().items()}
+    inputs = {k: v.clone() for k, v in batch.items() if torch.is_tensor(v)}
+    metrics = collections.defaultdict(list)
+    ppo._update_from_batch(batch, 0, None, metrics)
+    out = dict(inputs=inputs, heads=heads, metrics={k: float(torch.as_tensor(v[0]).detach()) for k, v in metrics.items()})
+    torch.save(out, os.path.join(HERE, "ppo_loss.pt"))
+    print("ppo_loss", out["metrics"])
+
+
 def main():
     R = ref_shim.ref()
     torch.set_num_threads(8)
     only = sys.argv[1:]
+    if not only or "ppo_loss" in only:
+        _ppo_loss_case(R)
+        if only == ["ppo_loss"]:
+            return
     for name, c in CASES.items():
         if only and name not in only:
             continue

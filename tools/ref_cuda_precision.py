@@ -1,6 +1,6 @@
 """Runs on the GPU box: how far is the REFERENCE's own CUDA path (cuDNN TF32 convolutions, torch defaults) from its
 fp32 CPU path?  Same minibatch as tests/golden/bench128.pt (T=128 x 8 envs = 1024 frames of 256x256 RGB-D), unmodified
-reference classes from baseline/_ref, per-tensor gradient cosine / norm ratio of device=cuda vs device=cpu.
+reference classes from oracle/_ref, per-tensor gradient cosine / norm ratio of device=cuda vs device=cpu.
 Writes gpurun_out/ref_cuda_precision.json -- the yardstick the hb200 precision bars are read against."""
 import json
 import os
